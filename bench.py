@@ -66,7 +66,17 @@ def parse_args():
     ap.add_argument('--gather-every', type=int, default=0,
                     help='all-gather the episode metrics every this many steps (0 = once per scripted segment, i.e. per batch of rollouts)')
     ap.add_argument('--no-batched-env', action='store_true', help='skip the BatchedRampJobPartitioningEnvironment secondary figure')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned to its caller (rank 0) as DIR/step_stats.npy [B, STEP_STATS_LEN] '
+                         'and DIR/cluster_steps.npy [B], float64; the inputs are a function of the arguments, so two builds can '
+                         'be compared output for output')
     return ap.parse_args()
+
+
+def dump_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f'{name}.npy'), a)
 
 
 def usable_cores():
@@ -455,6 +465,10 @@ def run_b200_arm(args, rank, world, local_rank):
     t_wall = time.perf_counter() - t_wall0
     dev_ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if sampler else None
+    # the buffers are written again by the legs below: keep the last timed step's outputs now
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'step_stats': stats_dev.cpu().numpy().astype(np.float64),
+                                         'cluster_steps': ncs_dev.cpu().numpy().astype(np.float64)})
     launches = eng.launch_count - launches0
     kt = eng.lookahead_kernel_time(reset=True)
     fold_memo()

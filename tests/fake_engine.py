@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE: the subset of ``ddls_b200.engine.RampEngine`` the drop-in cluster environment uses, answered by the
-CPU oracle (oracle/ramp_oracle.c).  Lets the host-side logic of ``ddls_b200.host.RampClusterEnvironment`` be driven by the
-reference's own RampJobPartitioningEnvironment and agents where there is no GPU (tests/test_reference_dropin.py); the same
-test runs against the CUDA engine under ``-m gpu``.  Never imported by the product."""
+CPU oracle (oracle/ramp_oracle.c).  Lets the host-side logic of ``ddls_b200.host.RampClusterEnvironment`` be driven the way
+the reference's own RampJobPartitioningEnvironment and agents drive it where there is no GPU (tests/test_reference_dropin.py);
+the same test runs against the CUDA engine under ``-m gpu``.  Never imported by the product."""
 import copy
 
 import numpy as np

@@ -3,10 +3,16 @@
 RJPE:199-206), on one of the seeded golden episodes, and prints what the reference itself recorded for that episode
 (tests/golden/<case>.npz) next to what this run produced.
 
-    PYTHONHASHSEED=0 python tests/ref_dropin_driver.py <case> [--fake-engine]
+    PYTHONHASHSEED=0 python tests/ref_dropin_driver.py <case> [--fake-engine] [--reference-cluster] [--record PATH]
 
 --fake-engine answers the engine calls with the CPU oracle (tests/fake_engine.py) so the host logic can be checked
-without a GPU; without it the CUDA engine is used (needs cuda:0)."""
+without a GPU; without it the CUDA engine is used (needs cuda:0).  --reference-cluster runs the reference's own cluster
+environment instead of the drop-in.  Needs the reference checkout, so the suite does not run it; it regenerates the
+fixtures the suite replays:
+
+    PYTHONHASHSEED=0 python tests/ref_dropin_driver.py <case> --fake-engine --record tests/golden/dropin/<case>.npz
+    PYTHONHASHSEED=0 python tests/ref_dropin_driver.py <case> --fake-engine --reference-cluster   # RESULT line ->
+                                                                              # tests/golden/dropin/<case>_reference.json"""
 import json
 import os
 import random
@@ -34,12 +40,117 @@ EXTRA_CASES = {
 }
 
 
+class _RecordingGenerator:
+    """Wraps the reference's JobsGenerator: every job, gap and len() answer the drop-in receives is recorded."""
+
+    def __init__(self, gen, rec):
+        self._gen, self._rec = gen, rec
+
+    def __len__(self):
+        n = len(self._gen)
+        self._rec.gen_len.append(n)
+        return n
+
+    def sample_job(self):
+        job = self._gen.sample_job()
+        self._rec.draws.append(job)
+        return job
+
+    def sample_interarrival_time(self, size=None):
+        gap = self._gen.sample_interarrival_time(size=size)
+        self._rec.gaps.append(float(gap))
+        return gap
+
+    def __getattr__(self, name):
+        return getattr(self._gen, name)
+
+
+class SessionRecorder:
+    """Records what the reference hands to the drop-in cluster environment in the last episode (reset onwards) as a
+    session for tests/dropin_replay.py: jobs and gaps drawn, len(jobs_generator) answers, and per step the lowered Action
+    with its global worker / channel ids.  Lowered jobs already in the case's golden fixture are referred to by index."""
+
+    def __init__(self, base, shape):
+        from ddls_b200.lowering import ModelRegistry
+        from golden_io import Golden
+        self.base, self.shape = base, shape
+        self.models = ModelRegistry()
+        self.known = list(Golden(base).templates) if base else []
+        self.extra = []
+        self._clear()
+
+    def _clear(self):
+        self.gen_len, self.draws, self.gaps, self.steps, self.reset_args = [], [], [], [], None
+
+    def _tid(self, lj):
+        key = (lj.fingerprint(), lj.degree)
+        for i, t in enumerate(self.known + self.extra):
+            if (t.fingerprint(), t.degree) == key:
+                return i
+        self.extra.append(lj)
+        return len(self.known) + len(self.extra) - 1
+
+    def install(self, cls):
+        from ddls_b200.lowering import lower_job
+        rec, orig_reset, orig_step = self, cls.reset, cls.step
+
+        def reset(cluster, jobs_config, max_simulation_run_time=float('inf'), job_queue_capacity=10, seed=None, verbose=False):
+            if isinstance(jobs_config, dict):
+                from ddls.demands.jobs.jobs_generator import JobsGenerator
+                jobs_config = JobsGenerator(**jobs_config)
+            rec._clear()
+            rec.reset_args = (float(max_simulation_run_time), int(job_queue_capacity))
+            return orig_reset(cluster, _RecordingGenerator(jobs_config, rec), max_simulation_run_time, job_queue_capacity, seed, verbose)
+
+        def step(cluster, action, verbose=False):
+            entry = {'tid': -1}
+            job_ids = list(action.job_ids)
+            if len(job_ids) == 1:
+                lj = lower_job(cluster, action, job_ids[0], rec.models)        # before the step mounts the job
+                pjob = action.actions['op_partition'].partitioned_jobs[job_ids[0]]
+                entry = {'tid': rec._tid(lj), 'job_id': int(job_ids[0]), 'mount': lj.mount, 'workers': list(lj.worker_ids),
+                         'channels': list(lj.channel_ids), 'seq_time': float(pjob.details['job_sequential_completion_time']['A100'])}
+            rec.steps.append(entry)
+            return orig_step(cluster, action, verbose=verbose)
+
+        cls.reset, cls.step = reset, step
+
+    def save(self, path, n_env_steps, actions):
+        out = {'base': np.array(self.base), 'shape': np.array(self.shape, dtype=np.int64), 'reset': np.array(self.reset_args),
+               'gen_len': np.array(self.gen_len, dtype=np.int64), 'n_env_steps': np.array(n_env_steps),
+               'actions': np.array(actions, dtype=np.int64)}
+        assert len(self.gaps) == len(self.draws)
+        out['draw_job_id'] = np.array([int(j.job_id) for j in self.draws], dtype=np.int64)
+        out['draw_model'] = np.array([str(j.details['model']) for j in self.draws])
+        out['draw_f'] = np.array([[gap, j.original_job.details['job_total_op_memory_cost'], j.original_job.details['job_total_dep_size'],
+                                   j.details['job_sequential_completion_time']['A100'], j.details['max_acceptable_job_completion_time']['A100'],
+                                   j.max_acceptable_job_completion_time_frac, j.num_training_steps]
+                                  for j, gap in zip(self.draws, self.gaps)], dtype=np.float64).reshape(-1, 7)
+        out['step_tid'] = np.array([e['tid'] for e in self.steps], dtype=np.int32)
+        out['step_job_id'] = np.array([e.get('job_id', -1) for e in self.steps], dtype=np.int64)
+        out['step_seq_time'] = np.array([e.get('seq_time', 0.0) for e in self.steps], dtype=np.float64)
+        out['step_mount'] = np.array([[e['mount'].max_acceptable_jct, e['mount'].part_op_mem, e['mount'].part_dep_size, e['mount'].flow_size,
+                                       e['mount'].n_mounted_workers, e['mount'].n_mounted_channels] if e['tid'] >= 0 else [0.0] * 6
+                                      for e in self.steps], dtype=np.float64)
+        for key in ('workers', 'channels'):
+            lists = [e.get(key, []) for e in self.steps]
+            out[f'step_{key}'] = np.array([str(x) for lst in lists for x in lst])
+            out[f'step_{key}_ptr'] = np.concatenate([[0], np.cumsum([len(lst) for lst in lists])]).astype(np.int64)
+        out['n_extra'] = np.array(len(self.extra))
+        for i, lj in enumerate(self.extra):
+            out.update(lj.to_npz_dict(prefix=f'x{i}_'))
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        np.savez_compressed(path, **out)
+
+
 def main():
     case = sys.argv[1]
     fake = '--fake-engine' in sys.argv
     use_reference_cluster = '--reference-cluster' in sys.argv      # run the reference's own cluster environment instead
+    record_path = sys.argv[sys.argv.index('--record') + 1] if '--record' in sys.argv else None
     from oracle import ref_shim
     ref_shim.install()
+    from dropin_replay import cluster_result
     from oracle import gen_golden                     # CASES / make_env / the reference imports (no recording here)
     import ddls.environments.ramp_job_partitioning.ramp_job_partitioning_environment as rjpe_mod
     from ddls.distributions.uniform import Uniform
@@ -62,6 +173,11 @@ def main():
         spec.update(extra)
     else:
         spec = gen_golden.CASES[case]
+    recorder = None
+    if record_path is not None:
+        assert not use_reference_cluster
+        recorder = SessionRecorder('' if case in EXTRA_CASES else case, spec['shape'])
+        recorder.install(host_cluster.RampClusterEnvironment)
     seed = spec['seed']
     np.random.seed(seed)
     random.seed(seed)
@@ -95,34 +211,10 @@ def main():
         actions.append(int(a))
         obs, _, done, _ = env.step(int(a))
         n_env_steps += 1
-    cluster = env.cluster
-    es = cluster.episode_stats
-    out = {'n_env_steps': n_env_steps, 'actions': actions, 'using_reference_classes': bool(host.USING_REFERENCE_CLASSES),
-           'n_cluster_steps': len(cluster.steps_log['step_end_time']),
-           'completed_job_idxs': [int(k) for k in cluster.jobs_completed.keys()],
-           'blocked_job_idxs': [int(k) for k in cluster.jobs_blocked.keys()],
-           'steps_log': {k: [float(x) for x in cluster.steps_log[k]] for k in
-                         ('step_start_time', 'step_end_time', 'num_jobs_completed', 'num_jobs_arrived', 'num_jobs_blocked',
-                          'mean_num_jobs_running', 'mean_compute_overhead_frac', 'mean_communication_overhead_frac',
-                          'compute_info_processed', 'mean_cluster_throughput')},
-           # the two step statistics the reference leaves as per-tick lists (RCE:989-994)
-           'tick_lists': {k: [[float(x) for x in step] for step in cluster.steps_log[k]] for k in
-                          ('mean_mounted_worker_utilisation_frac', 'mean_cluster_worker_utilisation_frac')}}
-    for k in ('num_jobs_arrived', 'num_jobs_completed', 'num_jobs_blocked'):
-        out[k] = int(es[k])
-    for k in ('episode_end_time', 'mean_load_rate', 'blocking_rate', 'acceptance_rate', 'compute_info_processed', 'dep_info_processed',
-              'flow_info_processed', 'cluster_info_processed', 'mean_compute_throughput', 'mean_cluster_throughput',
-              'mean_compute_overhead_frac', 'mean_communication_overhead_frac', 'mean_num_jobs_running', 'mean_num_mounted_workers'):
-        out[k] = float(es[k])
-    for k in ('job_completion_time', 'job_completion_time_speedup', 'job_communication_overhead_time', 'job_computation_overhead_time',
-              'jobs_completed_mean_mounted_worker_utilisation_frac', 'jobs_completed_num_mounted_workers',
-              'jobs_completed_num_mounted_channels', 'jobs_completed_max_acceptable_job_completion_time',
-              'jobs_blocked_max_acceptable_job_completion_time'):
-        out[k] = [float(x) for x in es[k]]
-    memo = cluster.job_model_to_max_num_partitions_to_init_details
-    out['is_dropin'] = not use_reference_cluster
-    out['last_step_stats'] = {k: float(cluster.step_stats[k]) for k in ('num_jobs_blocked', 'num_jobs_completed', 'num_jobs_arrived', 'step_end_time')}
-    out['init_details_memo_keys'] = sorted([str(m), int(p)] for m in memo for p in memo[m])
+    out = cluster_result(env.cluster, n_env_steps, actions, is_dropin=not use_reference_cluster,
+                         using_reference_classes=host.USING_REFERENCE_CLASSES)
+    if recorder is not None:
+        recorder.save(record_path, n_env_steps, actions)
     print('RESULT ' + json.dumps(out), flush=True)
 
 

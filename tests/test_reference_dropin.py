@@ -1,12 +1,14 @@
-"""The drop-in ``ddls_b200.host.RampClusterEnvironment`` inside the UNMODIFIED reference: RampJobPartitioningEnvironment
-(RJPE:199-206 swapped to the drop-in), the reference's own first-fit placers, SRPT schedulers, Job and JobsGenerator classes,
-on the seeded golden episodes -- the per-step log and the episode statistics must equal what the reference recorded for
-itself (tests/golden/*.npz, written by oracle/gen_golden.py).
+"""The drop-in ``ddls_b200.host.RampClusterEnvironment`` driven the way the UNMODIFIED reference drives it: its
+RampJobPartitioningEnvironment (RJPE:199-206 swapped to the drop-in), first-fit placers, SRPT schedulers, Job and
+JobsGenerator classes, on the seeded golden episodes.  Everything the reference handed to the drop-in in those episodes is
+stored as a session (tests/golden/dropin/<case>.npz, recorded by tests/ref_dropin_driver.py --record) and replayed by
+tests/dropin_replay.py; the per-step log and the episode statistics must equal what the reference recorded for itself
+(tests/golden/<case>.npz, written by oracle/gen_golden.py), or what the reference's own cluster environment produced on the
+same episode (tests/golden/dropin/<case>_reference.json, tests/ref_dropin_driver.py --reference-cluster).
 
-Needs the reference: the checkout in the build container, or the copy staged at oracle/_ref (oracle/stage_ref.py) on the
-GPU box.  The CPU variant answers the engine calls with the oracle (tests/fake_engine.py): it checks the HOST logic
-(mount bookkeeping, lowering of the reference's real Action objects, arrival streaming, replay into episode_stats, the
-init-details memo).  The ``-m gpu`` variant is the same run on the CUDA engine."""
+The CPU variant answers the engine calls with the oracle (tests/fake_engine.py): it checks the HOST logic (mount
+bookkeeping, lowering of reference-shaped Action objects, arrival streaming, replay into episode_stats, the init-details
+memo).  The ``-m gpu`` variant is the same run on the CUDA engine."""
 import json
 import os
 import subprocess
@@ -23,19 +25,19 @@ CASES = ['chain8', 'chain8_busy', 'chain8_maxtime', 'mixed16', 'res16_flood', 'r
          'resnet32_cfg2']         # BASELINE config 2's cluster and job (32 workers, ResNet-50-like), degrees 4 / 6 / 8
 
 
-def _reference_available():
-    from oracle import ref_shim
-    return ref_shim.reference_available()
-
-
-def _run(case, fake, reference_cluster=False):
-    cmd = [sys.executable, os.path.join(ROOT, 'tests', 'ref_dropin_driver.py'), case] + (['--fake-engine'] if fake else [])
-    if reference_cluster:
-        cmd.append('--reference-cluster')
+def _run(case, fake):
+    """The drop-in's result on the recorded session of ``case``."""
+    cmd = [sys.executable, os.path.join(ROOT, 'tests', 'dropin_replay.py'), case] + (['--fake-engine'] if fake else [])
     p = subprocess.run(cmd, capture_output=True, text=True, timeout=1500, env=dict(os.environ, PYTHONHASHSEED='0'))
     lines = [l for l in p.stdout.splitlines() if l.startswith('RESULT ')]
     assert p.returncode == 0 and lines, (p.stdout[-2000:], p.stderr[-4000:])
     return json.loads(lines[-1][len('RESULT '):])
+
+
+def _reference_result(case):
+    """The reference's own cluster environment on the same episode (recorded live)."""
+    with open(os.path.join(ROOT, 'tests', 'golden', 'dropin', f'{case}_reference.json')) as f:
+        return json.load(f)
 
 
 def _check(case, out):
@@ -79,8 +81,6 @@ def _check(case, out):
 
 @pytest.mark.parametrize('case', CASES)
 def test_dropin_inside_the_reference_host_logic(case):
-    if not _reference_available():
-        pytest.skip('reference not available (neither the build container checkout nor oracle/_ref)')
     out = _run(case, fake=True)
     _check(case, out)
 
@@ -88,8 +88,6 @@ def test_dropin_inside_the_reference_host_logic(case):
 @pytest.mark.gpu
 @pytest.mark.parametrize('case', CASES)
 def test_dropin_inside_the_reference_on_cuda(case):
-    if not _reference_available():
-        pytest.skip('reference not staged at oracle/_ref')
     out = _run(case, fake=False)
     _check(case, out)
 
@@ -120,9 +118,7 @@ def test_per_tick_utilisation_lists_equal_the_reference(case):
     """step_stats['mean_mounted_worker_utilisation_frac'] / ['mean_cluster_worker_utilisation_frac'] stay per-tick lists in the
     reference (RCE:989-994); the drop-in returns the engine's own per-iteration entries (every event ends the reference's step --
     RCE:1003-1044 -- so a list has one entry unless rounding keeps an event from firing; the engine records however many there are)."""
-    if not os.path.isdir('/root/' + 'reference'):
-        pytest.skip('needs the build container: runs the reference live for comparison')
-    ref = _run(case, fake=True, reference_cluster=True)
+    ref = _reference_result(case)
     mine = _run(case, fake=True)
     assert all(len(step) >= 1 for step in ref['tick_lists']['mean_mounted_worker_utilisation_frac'])
     _check_live(mine, ref)
@@ -132,9 +128,7 @@ def test_per_tick_utilisation_lists_equal_the_reference(case):
 def test_dropin_with_a_generator_that_never_runs_dry(case):
     """'remove_and_repeat' sampling: len(jobs_generator) never reaches 0, the episode ends on max_simulation_run_time and jobs
     keep arriving until then -- the drop-in streams arrivals one ahead instead of fixing their number at reset."""
-    if not os.path.isdir('/root/' + 'reference'):
-        pytest.skip('needs the build container: runs the reference live for comparison')
-    ref = _run(case, fake=True, reference_cluster=True)
+    ref = _reference_result(case)
     mine = _run(case, fake=True)
     assert ref['num_jobs_arrived'] > 6            # more arrivals than the 3 / 2 distinct jobs the generator holds
     _check_live(mine, ref)
@@ -143,8 +137,6 @@ def test_dropin_with_a_generator_that_never_runs_dry(case):
 @pytest.mark.gpu
 @pytest.mark.parametrize('case', ['chain8_repeat'])
 def test_dropin_with_a_generator_that_never_runs_dry_on_cuda(case):
-    if not _reference_available():
-        pytest.skip('reference not staged at oracle/_ref')
-    ref = _run(case, fake=True, reference_cluster=True)
+    ref = _reference_result(case)
     mine = _run(case, fake=False)
     _check_live(mine, ref)
