@@ -121,6 +121,8 @@ def lib():
                                              C.c_void_p, C.c_void_p, C.c_int32]
         L.orc_run_scripted_rjpe_batch.restype = C.c_int
         L.orc_run_scripted_rjpe_batch.argtypes = L.orc_run_scripted_batch.argtypes
+        L.orc_run_scripted_rjpe_batch_ex.restype = C.c_int
+        L.orc_run_scripted_rjpe_batch_ex.argtypes = L.orc_run_scripted_batch.argtypes[:-1] + [C.c_void_p, C.c_int32]
         _lib = L
     return _lib
 
@@ -159,6 +161,37 @@ def utilisation(trace_n_active, trace_tick, n_mounted_workers, jct):
     tn = np.ascontiguousarray(trace_n_active, dtype=np.int32)
     tt = np.ascontiguousarray(trace_tick, dtype=np.float64)
     return lib().orc_utilisation(tn.ctypes.data, tt.ctypes.data, len(tn), n_mounted_workers, jct)
+
+
+def run_scripted(templates, script_tid, script_mount, arrivals, n_workers, n_models, n_threads=None,
+                 max_simulation_run_time=float('inf')):
+    """B independent scripted episodes of L RampJobPartitioningEnvironment.step calls each (RJPE:300-420), one oracle env per
+    episode, spread over ``n_threads`` host threads.  Env-step s of episode b mounts ``templates[script_tid[b, s]]`` with the
+    mount scalars ``script_mount[b, s]`` (MOUNT_DTYPE) when a job is queued, else (or when the id is -1) is Action(); then
+    Action() steps follow until a job is queued or the episode is done.
+
+    Returns (stats [B, L, STEP_STATS_LEN] f64: the action step's statistics with `done` after the whole env-step,
+    records [B, J] JOB_RECORD_DTYPE, cluster_steps [B, L] int32: RampClusterEnvironment.step calls of each env-step)."""
+    tid = np.ascontiguousarray(script_tid, dtype=np.int32)
+    B, L = tid.shape
+    mount = np.ascontiguousarray(script_mount, dtype=MOUNT_DTYPE)
+    arr = np.ascontiguousarray(arrivals, dtype=ARRIVAL_DTYPE)
+    assert mount.shape == (B, L) and arr.ndim == 2 and arr.shape[0] == B
+    J = arr.shape[1]
+    keep = [to_c(t) for t in templates]                      # the structs point into the templates' arrays
+    ctemps = (CLoweredJob * max(len(keep), 1))(*keep)
+    stats = np.zeros((B, L, STEP_STATS_LEN), dtype=np.float64)
+    records = np.zeros((B, J), dtype=JOB_RECORD_DTYPE)
+    ncs = np.zeros((B, L), dtype=np.int32)
+    if n_threads is None:
+        n_threads = len(os.sched_getaffinity(0))
+    rc = lib().orc_run_scripted_rjpe_batch_ex(ctemps, len(keep), B, L, tid.ctypes.data, mount.ctypes.data, arr.ctypes.data, J,
+                                              float(max_simulation_run_time), int(n_workers), int(n_models), 1025,
+                                              stats.ctypes.data, records.ctypes.data, ncs.ctypes.data, int(n_threads))
+    if rc != 0:
+        raise Exception(f'orc_run_scripted_rjpe_batch_ex failed with status {rc}')
+    del keep
+    return stats, records, ncs
 
 
 class OracleEnv:

@@ -52,7 +52,7 @@ int orc_run_lookahead_batch(const orc_lowered_job_t* const* jobs, int32_t n,
 typedef struct {
     const orc_lowered_job_t* templates; int32_t n_templates, n_steps, n_jobs, n_cluster_workers, memo_models, memo_degrees;
     const int32_t* script_tid; const orc_mount_t* script_mount; const orc_arrival_t* arrivals;
-    double max_sim_time; double* stats_out; orc_job_record_t* records_out; atomic_int bad; int rjpe;
+    double max_sim_time; double* stats_out; orc_job_record_t* records_out; int32_t* ncs_out; atomic_int bad; int rjpe;
 } orc_sb_t;
 static void orc_sb_body(int32_t b, void* c) {
     orc_sb_t* x = (orc_sb_t*)c;
@@ -72,14 +72,17 @@ static void orc_sb_body(int32_t b, void* c) {
         else
             rc = orc_env_step(env, NULL, NULL, st);
         if (rc != ORC_OK) bad = 1;
+        int32_t n_cluster_steps = 1;
         if (x->rjpe) {   /* RJPE:394-395: while len(job_queue) == 0 and not done: step(Action()) */
             const double* last = st;
             while (!bad && orc_env_queued_job(env) < 0 && last[SS_DONE] == 0.0) {
                 if (orc_env_step(env, NULL, NULL, scratch) != ORC_OK) bad = 1;
                 last = scratch;
+                ++n_cluster_steps;
             }
             st[SS_DONE] = last[SS_DONE];
         }
+        if (x->ncs_out) x->ncs_out[idx] = n_cluster_steps;
     }
     if (x->records_out)
         memcpy(x->records_out + (size_t)b * (size_t)x->n_jobs, orc_env_job_records(env), sizeof(orc_job_record_t) * (size_t)x->n_jobs);
@@ -97,25 +100,37 @@ int orc_run_scripted_batch(const orc_lowered_job_t* templates, int32_t n_templat
     x.templates = templates; x.n_templates = n_templates; x.n_steps = n_steps; x.n_jobs = n_jobs;
     x.n_cluster_workers = n_cluster_workers; x.memo_models = memo_models; x.memo_degrees = memo_degrees;
     x.script_tid = script_tid; x.script_mount = script_mount; x.arrivals = arrivals; x.max_sim_time = max_sim_time;
-    x.stats_out = stats_out; x.records_out = records_out; atomic_init(&x.bad, 0); x.rjpe = 0;
+    x.stats_out = stats_out; x.records_out = records_out; x.ncs_out = NULL; atomic_init(&x.bad, 0); x.rjpe = 0;
     orc_parallel_for(n_episodes, n_threads, orc_sb_body, &x);
     return atomic_load(&x.bad) ? ORC_ERR_BAD_ARG : ORC_OK;
 }
 
 /* Same, but each scripted decision is one RampJobPartitioningEnvironment.step (RJPE:300-420): the action step
  * followed by Action() steps until a job is queued or the episode is done.  stats_out rows describe the action
- * step (with SS_DONE = done after the whole env-step). */
+ * step (with SS_DONE = done after the whole env-step).  ncs_out [n_episodes][n_steps] (may be NULL): the number of
+ * RampClusterEnvironment.step calls each env-step made, the action step included. */
+int orc_run_scripted_rjpe_batch_ex(const orc_lowered_job_t* templates, int32_t n_templates,
+                                   int32_t n_episodes, int32_t n_steps,
+                                   const int32_t* script_tid, const orc_mount_t* script_mount,
+                                   const orc_arrival_t* arrivals, int32_t n_jobs,
+                                   double max_sim_time, int32_t n_cluster_workers, int32_t memo_models, int32_t memo_degrees,
+                                   double* stats_out, orc_job_record_t* records_out, int32_t* ncs_out, int32_t n_threads) {
+    orc_sb_t x;
+    x.templates = templates; x.n_templates = n_templates; x.n_steps = n_steps; x.n_jobs = n_jobs;
+    x.n_cluster_workers = n_cluster_workers; x.memo_models = memo_models; x.memo_degrees = memo_degrees;
+    x.script_tid = script_tid; x.script_mount = script_mount; x.arrivals = arrivals; x.max_sim_time = max_sim_time;
+    x.stats_out = stats_out; x.records_out = records_out; x.ncs_out = ncs_out; atomic_init(&x.bad, 0); x.rjpe = 1;
+    orc_parallel_for(n_episodes, n_threads, orc_sb_body, &x);
+    return atomic_load(&x.bad) ? ORC_ERR_BAD_ARG : ORC_OK;
+}
+
 int orc_run_scripted_rjpe_batch(const orc_lowered_job_t* templates, int32_t n_templates,
                                 int32_t n_episodes, int32_t n_steps,
                                 const int32_t* script_tid, const orc_mount_t* script_mount,
                                 const orc_arrival_t* arrivals, int32_t n_jobs,
                                 double max_sim_time, int32_t n_cluster_workers, int32_t memo_models, int32_t memo_degrees,
                                 double* stats_out, orc_job_record_t* records_out, int32_t n_threads) {
-    orc_sb_t x;
-    x.templates = templates; x.n_templates = n_templates; x.n_steps = n_steps; x.n_jobs = n_jobs;
-    x.n_cluster_workers = n_cluster_workers; x.memo_models = memo_models; x.memo_degrees = memo_degrees;
-    x.script_tid = script_tid; x.script_mount = script_mount; x.arrivals = arrivals; x.max_sim_time = max_sim_time;
-    x.stats_out = stats_out; x.records_out = records_out; atomic_init(&x.bad, 0); x.rjpe = 1;
-    orc_parallel_for(n_episodes, n_threads, orc_sb_body, &x);
-    return atomic_load(&x.bad) ? ORC_ERR_BAD_ARG : ORC_OK;
+    return orc_run_scripted_rjpe_batch_ex(templates, n_templates, n_episodes, n_steps, script_tid, script_mount, arrivals, n_jobs,
+                                          max_sim_time, n_cluster_workers, memo_models, memo_degrees, stats_out, records_out,
+                                          NULL, n_threads);
 }

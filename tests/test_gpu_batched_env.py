@@ -2,7 +2,8 @@
 one engine, every decision lowered by the native placer + native expansion (no reference objects) -- replays the reference's
 recorded golden episodes SIDE BY SIDE in one batch: same arrival streams, same actions (the partition degrees the reference's
 actors chose), and must reproduce what the reference recorded for each episode: the statistics of every env-step's first
-cluster step, which jobs completed / were blocked, every job completion time and overhead (<= 1e-6 relative)."""
+cluster step, which jobs completed / were blocked, every job completion time and overhead (<= 1e-6 relative), and every
+env-step's reward against the reference's rule evaluated on the CPU oracle replaying the same episode."""
 import numpy as np
 import pytest
 
@@ -105,6 +106,15 @@ def test_batched_env_replays_reference_episodes_in_lock_step(names, where):
     obs = env.reset()
     for b, g in enumerate(goldens):
         env.eng.set_job_count(b, len(g.d['arrivals']))
+    # each golden episode replayed on the CPU oracle beside the batch: it says whether a placed job was blocked by the end of its
+    # action's cluster step, which is what the reference's reward looks at (RJPE:379-391, rewards/job_acceptance.py)
+    from oracle import oracle
+    oracle.build()
+    oenvs = []
+    for g in goldens:
+        oe = oracle.OracleEnv(g.n_cluster_workers, max_jobs=len(g.arrivals()), memo_models=max(g.n_models, 1))
+        oe.reset(g.arrivals(), max_simulation_run_time=g.max_sim_time)
+        oenvs.append(oe)
     n_env_steps = max(len(d) for d in decisions)
     exact = ['num_jobs_completed', 'num_jobs_arrived', 'num_jobs_blocked']
     close = ['step_start_time', 'step_end_time', 'mean_num_jobs_running', 'mean_compute_overhead_frac', 'mean_communication_overhead_frac',
@@ -115,14 +125,13 @@ def test_batched_env_replays_reference_episodes_in_lock_step(names, where):
             if e < len(decisions[b]):
                 assert not env.done[b], (names[b], e)
                 assert env.queued[b] == e
-                a = decisions[b][e][1]
-                assert a == 0 or obs['action_mask'][b, a] == 1 or True
-                actions[b] = a
+                actions[b] = decisions[b][e][1]
             else:
                 assert env.done[b], (names[b], e)
         obs, reward, done, info = env.step(actions)
         for b, g in enumerate(goldens):
             if e >= len(decisions[b]):
+                assert reward[b] == 0.0, (names[b], e, reward[b])        # the episode was already done
                 continue
             s = decisions[b][e][0]
             ref = g.d['step_stats'][s]
@@ -131,8 +140,18 @@ def test_batched_env_replays_reference_episodes_in_lock_step(names, where):
                 assert st[SS[k]] == ref[SS[k]], (names[b], e, k, st[SS[k]], ref[SS[k]])
             for k in close:
                 assert st[SS[k]] == pytest.approx(ref[SS[k]], rel=1e-6, abs=0), (names[b], e, k)
-            # the reference's reward: +1 iff the job was placed and not blocked by its lookahead (rewards/job_acceptance.py)
+            # the reference's reward: success iff the decision placed the job and the job is not blocked after the action's
+            # cluster step, else fail (RJPE:379-391, rewards/job_acceptance.py)
             placed = decisions[b][e][1] > 0 and int(g.d['step_tid'][s]) >= 0
+            oe = oenvs[b]
+            assert oe.queued_job == e, (names[b], e, oe.queued_job)
+            o = oe.step(g.step_job(s) if placed else None)
+            blocked = oe.job_records()['status'][e] == JS_BLOCKED
+            want = env.success_reward if placed and not blocked else env.fail_reward
+            assert reward[b] == want, (where, names[b], e, 'placed' if placed else 'not placed', 'blocked' if blocked else '',
+                                       reward[b], want)
+            while oe.queued_job < 0 and o[SS['done']] == 0.0:                # RJPE:394-395
+                o = oe.step(None)
     assert env.done.all()
     rec = env.eng.job_records()
     for b, g in enumerate(goldens):
